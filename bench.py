@@ -11,6 +11,7 @@ interleaved over the ranks (the CS is recomputed per rank; no data-path
 collective); a strong-scaling leg over a fixed 8192-eta grid is reported too.
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference]
+                  [--dump-outputs DIR]
 
 The b200 arm reports device-resident throughput (`value`), end-to-end
 throughput through the public API with pinned host buffers (`e2e`), the
@@ -302,6 +303,25 @@ def collect_prof(L, _lib):
     return ms, cnt
 
 
+CS_SAMPLE = 1 << 20      # CS points written by --dump-outputs (8 MB)
+
+
+def dump_outputs(out_dir, buf, d_cs, ncols):
+    """What the last timed step computed, as DIR/<name>.npy: the sweep's per-eta
+    outputs in full (float64) and a fixed, seeded sample of the conjugate spectrum
+    (the fd >= 0 columns it computed; float32 [re, im] pairs), for comparing the
+    outputs of two builds run with the same arguments."""
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    for name in ("eigs", "stat", "nred", "iters"):
+        np.save(os.path.join(out_dir, name + ".npy"),
+                buf[name].cpu().numpy().astype(np.float64))
+    rng = np.random.default_rng(0)
+    rows = torch.from_numpy(rng.integers(0, d_cs.shape[0], CS_SAMPLE)).to(d_cs.device)
+    cols = torch.from_numpy(rng.integers(0, ncols, CS_SAMPLE)).to(d_cs.device)
+    np.save(os.path.join(out_dir, "cs_sample.npy"), d_cs[rows, cols].cpu().numpy())
+
+
 def b200_arm(args):
     import torch
     import torch.distributed as dist
@@ -401,6 +421,9 @@ def b200_arm(args):
     wbuf, wstep = make_leg(etas)
     ms_step, kern, launches, (wall0, wall1) = timed(wstep, args.warmup, args.steps)
     clk = clocks.stop(wall0, wall1)
+    if args.dump_outputs and rank == 0:
+        # before the strong leg, which reuses d_cs
+        dump_outputs(args.dump_outputs, wbuf, d_cs, keep or nfd // 2 + 1)
     value = world * NETA / (ms_step * 1e-3)
     eigs = wbuf["eigs"].cpu().numpy()
     nred = wbuf["nred"].cpu().numpy().astype(np.int64)
@@ -609,7 +632,12 @@ def main():
                     help="skip the strong-scaling leg (profiling runs)")
     ap.add_argument("--no-extra", action="store_true",
                     help="skip e2e_f64 and the C2/C4 extra configs (profiling runs)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one computed as "
+                         "DIR/<name>.npy (b200 arm; rank 0's share when --gpus > 1)")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs needs --impl b200")
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
     if args.impl == "reference":
         return reference_arm(args)

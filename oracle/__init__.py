@@ -34,3 +34,31 @@ Units convention of every unit-free function here: tau in us, fd / theta /
 edges in mHz, eta in s^3, time in s, freq in MHz.  eta*theta^2 is numerically
 already in us (s^3 * mHz^2 == 1e-6 s).
 """
+import hashlib
+
+import numpy as np
+
+
+def complex_digest(a):
+    """SHA-256 of ``a`` as C-ordered complex128 bytes.  Fixtures store this in place
+    of reference arrays too large to commit; equal digests mean bit-identical arrays."""
+    return hashlib.sha256(np.ascontiguousarray(a, dtype=np.complex128).tobytes()).hexdigest()
+
+
+def retrieval_maps(g):
+    """thth_red, rv_h and rv_n of the fixture tests/golden/retrieval_64x128.npz (``g``),
+    rebuilt by the oracle from the fixture's inputs and checked bit for bit against
+    the digests the fixture keeps of the reference's arrays."""
+    from oracle import thth_oracle as TO
+    eta = float(g["eta"])
+    CS = TO.conjugate_spectrum(g["d0"], int(g["npad"]), None)
+    out = {"thth_red": TO.thth_redmap(CS, g["tau"], g["fd"], eta, g["edges"])[0]}
+    n = out["thth_red"].shape[0]
+    rng = np.random.default_rng(int(g["tt_seed"]))
+    tt = rng.normal(size=(n, n)) + 1j * rng.normal(size=(n, n))
+    for herm, key in ((True, "rv_h"), (False, "rv_n")):
+        out[key] = TO.rev_map(tt, g["tau"], g["fd"], eta, g["edges_red"], hermetian=herm)
+    for key, a in out.items():
+        assert a.shape == tuple(g[key + "_shape"]), key
+        assert complex_digest(a) == str(g[key + "_sha256"]), key
+    return out

@@ -108,7 +108,8 @@ def test_thin_and_retrieval_fail_loudly_without_device(golden_dir):
     from scintools_b200 import ththmod
     g = np.load(os.path.join(golden_dir, "retrieval_64x128.npz"))
     with pytest.raises(RuntimeError):
-        ththmod.rev_map(g["thth_red"], g["tau"], g["fd"], float(g["eta"]), g["edges_red"])
+        ththmod.rev_map(np.ones(tuple(g["thth_red_shape"]), complex), g["tau"], g["fd"],
+                        float(g["eta"]), g["edges_red"])
     with pytest.raises(RuntimeError):
         ththmod.thin_sweep(np.zeros((256, 512), complex), g["tau"], g["fd"],
                            np.array([40.0]), g["edges"], g["edges"][60:200], 0.0)
